@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the HiFIC encode+decode forward hot path (Encoder -> Hyperprior -> Generator).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one pass of the hot path over one batch of B synthetic 3x256x256 images per GPU (weak scaling,
@@ -15,6 +15,8 @@ no data-path collective: samples are independent).  Prints ONE JSON line (rank 0
                 gradient all-reduce at N > 1), plus the same step with the native LPIPS trunk (single GPU)
   compress_path Model.compress / Model.decompress through the public API (GPU networks + symbol kernels + host rANS)
 `--impl reference` times the reference's CPU implementation of the path (oracle port) instead.
+`--dump-outputs DIR` writes what the last timed step returned (reconstruction, q_bpp) as DIR/<name>.npy, so that two builds
+can be compared output for output: weights and images are seeded, the inputs are the same on every run.
 """
 import argparse
 import json
@@ -705,6 +707,21 @@ def run_compress_path(model, dev, x_host):
     return out
 
 
+def dump_outputs(out_dir, outputs, rank, world, budget=64 << 20):
+    """Write each output tensor as out_dir/<name>.npy in float32 (`<name>_rank<r>.npy` at N > 1).  A tensor larger than
+    its share of `budget` is replaced by a fixed, seeded sample of its flattened elements (the same indices on every run
+    with the same arguments)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = budget // (world * len(outputs))
+    for name, t in outputs.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy" if world == 1 else f"{name}_rank{rank}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -722,6 +739,8 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from Python instead of replaying a CUDA graph")
     ap.add_argument("--profile", action="store_true",
                     help="profiling mode (ncu): device-resident steps only, no e2e / roofline / CPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
 
@@ -753,9 +772,12 @@ def main():
     out_host = torch.empty((B, 3, 256, 256), dtype=torch.float32).pin_memory()
     bpp_host = torch.empty((), dtype=torch.float32).pin_memory()
 
+    last = {}
+
     def step_device():
         with torch.no_grad():
-            return model(x_dev, writeout=False)
+            last["reconstruction"], last["q_bpp"] = model(x_dev, writeout=False)
+            return last["reconstruction"], last["q_bpp"]
 
     # end to end through the public API with HOST buffers: every step copies its input from pinned host memory and
     # its result back; hific_b200.pipeline.PipelinedForward double-buffers the copies on their own streams so that
@@ -804,6 +826,8 @@ def main():
     torch.cuda.synchronize()
     if args.profile:
         ms = timed(step_device, args.steps)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last, rank, world)
         if rank == 0:
             print(json.dumps({"profile_mode": True, "ms_per_step_under_profiler": ms / args.steps}))
         return
@@ -812,6 +836,8 @@ def main():
     if rank == 0:
         sampler.start()
     ms = timed(step_device, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last, rank, world)
     launches = launches_per_step * args.steps
     for _ in range(2):
         step_e2e()

@@ -1,7 +1,7 @@
-"""Import the UNMODIFIED reference (read-only, /root/reference) in this container -- TEST INFRASTRUCTURE.
+"""Import the UNMODIFIED reference (read-only, a checkout named by HIFIC_REFERENCE_ROOT) -- TEST INFRASTRUCTURE.
 
-Only usable where /root/reference exists (the build container); nothing that runs on the GPU box may import
-this.  Three workarounds, none touching hot-path arithmetic (SURVEY.md section 8c):
+Only usable where such a checkout exists; nothing that runs on a GPU machine may depend on it.  Three workarounds, none
+touching hot-path arithmetic (SURVEY.md section 8c):
   1. `autograd` (HIPS) is not installed: stubbed (only the host ANS coder uses it);
   2. `skimage` is not installed: stubbed (imported by LPIPS / datasets, unused on the path);
   3. no network: torchvision's `alexnet(pretrained=True)` becomes a seeded random trunk.
@@ -10,16 +10,16 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("HIFIC_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("HIFIC_REFERENCE_ROOT", "")
 
 
 def available():
-    return os.path.isdir(os.path.join(REF_ROOT, "src"))
+    return bool(REF_ROOT) and os.path.isdir(os.path.join(REF_ROOT, "src"))
 
 
 def install():
     if not available():
-        raise RuntimeError(f"reference not found at {REF_ROOT}")
+        raise RuntimeError(f"reference not found at HIFIC_REFERENCE_ROOT={REF_ROOT!r}")
     import numpy as np
     if "autograd" not in sys.modules:
         ag = types.ModuleType("autograd")
