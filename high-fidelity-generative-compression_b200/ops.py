@@ -663,3 +663,60 @@ class DlmmLikelihoodFn(torch.autograd.Function):
         dd = d_decoded.contiguous() if d_decoded is not None else None
         dx, dparams = dlmm_likelihood_bwd(x, dlmm_params, noise, dd, g, ctx.kind)
         return dx, dparams, None, None, None
+
+
+# ------------------------------------------------------------------------------------------------------------
+# PSNR / SSIM / MS-SSIM of the evaluation loop (csrc/ssim.cu; src/helpers/metrics.py)
+# ------------------------------------------------------------------------------------------------------------
+_metrics_ws_cache = {}
+
+
+def _metrics_ws(key, need, device):
+    """Scratch of the metric kernels, one buffer per (kind, device), grown on demand; the launches that use it are ordered
+    on the current stream."""
+    if need < 0:
+        raise _lib.HfcError(f"libhfc {key} workspace query failed: {lib.hfc_last_error().decode('utf-8', 'replace')}")
+    buf = _metrics_ws_cache.get((key, device))
+    if buf is None or buf.numel() * 8 < need:
+        buf = _metrics_ws_cache[(key, device)] = torch.empty(max(1, (need + 7) // 8), dtype=torch.float64, device=device)
+    return buf, buf.numel() * 8
+
+
+def ssim_levels(x, y, taps, c1, c2, weights, relu_last, size_average):
+    """x, y (N, C, H, W) fp32 CUDA; taps (C, win) fp32 on x's device.  len(weights) SSIM levels (2x2 average pool in
+    between) -> prod_l value_l ** weights[l] per plane, averaged over (N, C) (0-d tensor) or over C per image ((N,)).
+    len(weights) + 1 launches, no synchronisation."""
+    assert x.is_cuda and x.dtype == torch.float32 and x.dim() == 4 and y.shape == x.shape and y.dtype == x.dtype
+    x, y = x.contiguous(), y.contiguous()
+    n, c, h, w = x.shape
+    win = taps.shape[-1]
+    assert taps.is_cuda and taps.dtype == torch.float32 and taps.is_contiguous() and tuple(taps.shape) == (c, win)
+    levels = len(weights)
+    ws, ws_bytes = _metrics_ws("ssim", int(lib.hfc_ssim_ws_bytes(n, c, h, w, win, levels)), x.device)
+    for level in range(levels):
+        if level < levels - 1:
+            hp, wp = (x.shape[2] + 1) // 2, (x.shape[3] + 1) // 2
+            px = torch.empty((n, c, hp, wp), dtype=torch.float32, device=x.device)
+            py = torch.empty_like(px)
+        else:
+            px = py = None
+        check(lib.hfc_ssim_level(_ptr(x), _ptr(y), n, c, h, w, level, _ptr(taps), win, c1, c2, _ptr(px), _ptr(py),
+                                 _ptr(ws), ws_bytes, _stream()), "ssim_level")
+        x, y = px, py
+    out = torch.empty(1 if size_average else n, dtype=torch.float32, device=ws.device)
+    wts = (ctypes.c_float * levels)(*weights)
+    check(lib.hfc_ssim_finalize(n, c, h, w, win, levels, wts, int(bool(relu_last)), int(bool(size_average)), _ptr(ws),
+                                ws_bytes, _ptr(out), _stream()), "ssim_finalize")
+    return out.reshape(()) if size_average else out
+
+
+def psnr(a, b, max_val=255.0):
+    """a, b (N, ...) fp32 CUDA -> (N,) float64 per-image PSNR in dB (2 launches, no synchronisation)."""
+    assert a.is_cuda and a.dtype == torch.float32 and b.shape == a.shape and b.dtype == a.dtype and a.dim() >= 1
+    a, b = a.contiguous(), b.contiguous()
+    n = a.shape[0]
+    per_image = a.numel() // n
+    ws, ws_bytes = _metrics_ws("psnr", int(lib.hfc_psnr_ws_bytes(n, per_image)), a.device)
+    out = torch.empty(n, dtype=torch.float64, device=a.device)
+    check(lib.hfc_psnr(_ptr(a), _ptr(b), n, per_image, float(max_val), _ptr(ws), ws_bytes, _ptr(out), _stream()), "psnr")
+    return out

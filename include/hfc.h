@@ -460,6 +460,35 @@ int hfc_dlmm_likelihood_bwd(const float* x, const float* noise, const float* dlm
                             const float* g_nbpp, float coef, int32_t n, int32_t c, int32_t k, int32_t hw,
                             int32_t likelihood_type, float* dx, float* dparams, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------
+ * Image-quality metrics of the evaluation loop (compress.py --metrics), src/helpers/metrics.py.  x, y: fp32 NCHW
+ * (n, c, h, w), contiguous; all reductions run in a fixed order (no float atomics), so every result is bit-reproducible
+ * and an image's value does not depend on the rest of the batch.
+ *
+ * SSIM / MS-SSIM (metrics.py:37-63 gaussian_filter, 66-103 _ssim, 106-161 ssim, 164-236 ms_ssim): one hfc_ssim_level
+ * launch per level, then one hfc_ssim_finalize.  (h0, w0) is the level-0 size; level l's inputs are (n, c, h_l, w_l),
+ * h_{l+1} = (h_l + 1) / 2.  taps: (c, win) window taps per channel (odd win <= 31).  A dimension smaller than win is
+ * not smoothed (the reference's gaussian_filter skips it).  c1 = (K1 * data_range)^2, c2 = (K2 * data_range)^2.
+ * x_pooled / y_pooled: (n, c, h_{l+1}, w_{l+1}), the F.avg_pool2d(kernel 2, padding h_l % 2, w_l % 2) of x / y, the next
+ * level's inputs; both NULL at the last level.  ws: device scratch of at least hfc_ssim_ws_bytes(n, c, h0, w0, win,
+ * levels) bytes (8-byte aligned), shared by all levels of one call; it need not be initialised.
+ * hfc_ssim_finalize: per plane, the mean over each level's valid outputs, relu(cs) below the last level, the last level's
+ * ssim (relu'd when relu_last), prod_l value_l ** weights_host[l] (levels <= 8); out = the mean over all (n, c)
+ * (size_average, out[0]) or per image (out[0..n)).  ms_ssim: relu_last = 1; ssim: levels = 1, weight 1,
+ * relu_last = nonnegative_ssim.
+ * --------------------------------------------------------------------------------------------------------- */
+int64_t hfc_ssim_ws_bytes(int32_t n, int32_t c, int32_t h, int32_t w, int32_t win, int32_t levels);
+int hfc_ssim_level(const float* x, const float* y, int32_t n, int32_t c, int32_t h0, int32_t w0, int32_t level,
+                   const float* taps, int32_t win, float c1, float c2, float* x_pooled, float* y_pooled, void* ws,
+                   int64_t ws_bytes, void* stream);
+int hfc_ssim_finalize(int32_t n, int32_t c, int32_t h0, int32_t w0, int32_t win, int32_t levels, const float* weights_host,
+                      int32_t relu_last, int32_t size_average, void* ws, int64_t ws_bytes, float* out, void* stream);
+/* PSNR (metrics.py:7-18): out[i] = 20 log10(max_val) - 10 log10(mean over image i of (a - b)^2), fp64 throughout;
+ * per_image = c * h * w.  ws: device scratch of at least hfc_psnr_ws_bytes(n, per_image) bytes.  Two launches. */
+int64_t hfc_psnr_ws_bytes(int32_t n, int64_t per_image);
+int hfc_psnr(const float* a, const float* b, int32_t n, int64_t per_image, double max_val, void* ws, int64_t ws_bytes,
+             double* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
