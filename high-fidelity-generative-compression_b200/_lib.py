@@ -138,6 +138,13 @@ SIGNATURES = {
     "hfc_ssim_level": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _i32, _f32, _f32, _vp, _vp, _vp, _i64,
                                       _vp]),
     "hfc_ssim_finalize": (ctypes.c_int, [_i32, _i32, _i32, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _i64, _vp, _vp]),
+    "hfc_ssim_grad_maps_bytes": (ctypes.c_int64, [_i32, _i32, _i32, _i32, _i32, _i32]),
+    "hfc_ssim_grad_coeffs": (ctypes.c_int, [_i32, _i32, _i32, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _i64, _vp, _vp,
+                                            _vp]),
+    "hfc_ssim_grad_maps": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _i32, _f32, _f32, _vp, _vp,
+                                          _i64, _vp]),
+    "hfc_ssim_level_bwd": (ctypes.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp,
+                                          _vp]),
     "hfc_psnr_ws_bytes": (ctypes.c_int64, [_i32, _i64]),
     "hfc_psnr": (ctypes.c_int, [_vp, _vp, _i32, _i64, ctypes.c_double, _vp, _i64, _vp, _vp]),
 }

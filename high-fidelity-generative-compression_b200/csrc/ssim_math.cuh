@@ -1,6 +1,6 @@
 // Per-pixel, per-pooled-pixel and per-plane code of the SSIM / MS-SSIM kernels (csrc/ssim.cu).  Shared by the CUDA kernels
-// and by the host harness tests/ssim_math_host.cpp, which compiles THIS file with g++ so that the arithmetic, the tiling and
-// the pooling ownership the GPU runs are checked on the CPU.  Reference: src/helpers/metrics.py:37-63 (gaussian_filter),
+// and by the host harnesses tests/ssim_math_host.cpp (forward) and tests/ssim_grad_host.cpp (backward), which compile THIS
+// file with g++ so that the arithmetic, the tiling and the pooling ownership the GPU runs are checked on the CPU.  Reference: src/helpers/metrics.py:37-63 (gaussian_filter),
 // 66-103 (_ssim), 164-236 (ms_ssim).
 //
 // Every rounding step is explicit (mul_rn / add_rn / fmaf), so nvcc's FMA contraction cannot make the device differ from
@@ -154,5 +154,94 @@ HFC_HD float ssim_plane_value(const double* sums, const float* weights, int leve
   }
   return prod;
 }
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Backward (hfc_ssim_grad_coeffs / hfc_ssim_grad_maps / hfc_ssim_level_bwd)
+// ---------------------------------------------------------------------------------------------------------------------
+
+// One plane's per-level pixel coefficients from its per-level sums (as ssim_plane_value reads them) and the upstream
+// gradient dv of the plane value.  coef[2 l] = alpha_l = dV / dS_l / count_l (the weight of each output's ssim),
+// coef[2 l + 1] = beta_l = dV / dCS_l / count_l (the weight of each output's cs).  Level k's factor is f_k = v_k ** w_k;
+// its derivative is w_k v_k ** (w_k - 1) times the product of the OTHER factors, formed explicitly (never V / f_k).  A
+// level clamped by its relu (v_k <= 0) gets exactly 0, as torch's threshold_backward gives, and so does every level when
+// another is clamped (its factor is 0 in their products).  fp64 throughout, rounded to fp32 at the end.
+HFC_HD void ssim_grad_coeffs(const double* sums, const float* weights, int levels, int h0, int w0, int win,
+                             int relu_last, double dv, float* coef) {
+  float v[kSsimMaxLevels], f[kSsimMaxLevels];
+  for (int l = 0; l < levels; ++l) {
+    const SsimLevelGeom g = ssim_level_geom(h0, w0, win, l);
+    const double count = static_cast<double>(g.ho) * g.wo;
+    const bool last = l == levels - 1;
+    v[l] = static_cast<float>(sums[2 * l + (last ? 0 : 1)] / count);
+    if (!last || relu_last) v[l] = relu_keep_nan(v[l]);
+    f[l] = weights[l] == 1.f ? v[l] : powf(v[l], weights[l]);
+  }
+  for (int l = 0; l < levels; ++l) {
+    const SsimLevelGeom g = ssim_level_geom(h0, w0, win, l);
+    const double count = static_cast<double>(g.ho) * g.wo;
+    const bool last = l == levels - 1;
+    const bool masked = (!last || relu_last) && !(v[l] > 0.f);
+    double d = 0.0;
+    if (!masked) {
+      double others = 1.0;
+      for (int j = 0; j < levels; ++j)
+        if (j != l) others *= static_cast<double>(f[j]);
+      const double dpow = weights[l] == 1.f ? 1.0
+                                            : static_cast<double>(weights[l]) *
+                                                  pow(static_cast<double>(v[l]), static_cast<double>(weights[l]) - 1.0);
+      d = dv * others * dpow / count;
+    }
+    coef[2 * l] = last ? static_cast<float>(d) : 0.f;
+    coef[2 * l + 1] = last ? 0.f : static_cast<float>(d);
+  }
+}
+
+// Upstream gradient of plane p's value: grad_out[0] / (n c) when the output is the batch mean, else grad_out[image] / c.
+HFC_HD double ssim_grad_dv(const float* grad_out, int64_t p, int64_t planes, int c, int size_average) {
+  return size_average ? static_cast<double>(grad_out[0]) / static_cast<double>(planes)
+                      : static_cast<double>(grad_out[p / c]) / c;
+}
+
+// The four per-output gradient maps of a level, from the five filtered moments and the level's coefficients
+// (alpha: weight of ssim, beta: weight of cs):  gam = beta + alpha l, lam = alpha cs,
+//   gE = -gam cs / D (to exx and eyy), gXY = 2 gam / D,
+//   gmu1 = lam 2 (mu2 - l mu1) / B - 2 mu1 gE - mu2 gXY, gmu2 the same with 1 and 2 swapped.
+HFC_HD void ssim_grad_maps(float mu1, float mu2, float exx, float eyy, float exy, float c1, float c2, float alpha,
+                           float beta, float* gmu1, float* gmu2, float* ge, float* gxy) {
+  const float mu1_sq = mul_rn(mu1, mu1), mu2_sq = mul_rn(mu2, mu2), mu1_mu2 = mul_rn(mu1, mu2);
+  const float s1 = sub_rn(exx, mu1_sq), s2 = sub_rn(eyy, mu2_sq), s12 = sub_rn(exy, mu1_mu2);
+  const float D = add_rn(add_rn(s1, s2), c2);
+  const float B = add_rn(add_rn(mu1_sq, mu2_sq), c1);
+  const float cs = div_rn(add_rn(mul_rn(2.f, s12), c2), D);
+  const float l = div_rn(add_rn(mul_rn(2.f, mu1_mu2), c1), B);
+  const float gam = add_rn(beta, mul_rn(alpha, l));
+  const float lam = mul_rn(alpha, cs);
+  const float e = div_rn(mul_rn(-gam, cs), D);
+  const float xy = div_rn(mul_rn(2.f, gam), D);
+  const float lb = div_rn(mul_rn(2.f, lam), B);
+  *ge = e;
+  *gxy = xy;
+  *gmu1 = sub_rn(sub_rn(mul_rn(lb, sub_rn(mu2, mul_rn(l, mu1))), mul_rn(mul_rn(2.f, mu1), e)), mul_rn(mu2, xy));
+  *gmu2 = sub_rn(sub_rn(mul_rn(lb, sub_rn(mu1, mul_rn(l, mu2))), mul_rn(mul_rn(2.f, mu2), e)), mul_rn(mu1, xy));
+}
+
+// One input pixel's gradient from the adjoint-filtered maps (tmu = G^T gmu, te = G^T gE, txy = G^T gXY) and the pooled
+// gradient of the next level (0 at the last level): own = tmu + 2 x te + other txy, plus 0.25 * coarse.
+HFC_HD float ssim_grad_combine(float tmu, float te, float txy, float own, float other, float coarse) {
+  const float g = add_rn(add_rn(tmu, mul_rn(mul_rn(2.f, own), te)), mul_rn(other, txy));
+  return add_rn(g, mul_rn(0.25f, coarse));
+}
+
+// avg_pool2d(kernel 2, padding s % 2): input row i lies in pooled row (i + s % 2) / 2.
+HFC_HD int pooled_index_of(int i, int odd) { return (i + odd) >> 1; }
+
+// Level-backward tile: one CTA owns input tile (ty, tx) of kSsimTileH x kSsimTileW pixels of a level's input plane and
+// stages the four maps over output rows [r0 - (wh - 1), r0 + TH) and cols [c0 - (ww - 1), c0 + TW), zero outside the
+// valid outputs.  Staged row k is output row r0 - (wh - 1) + k; input row r0 + i reads staged rows i .. i + wh - 1 with
+// the flipped taps (the adjoint of the valid window is a full correlation with the taps reversed).
+HFC_HD int ssim_bwd_tiles_y(const SsimLevelGeom& g) { return ceil_div(g.h, kSsimTileH); }
+HFC_HD int ssim_bwd_tiles_x(const SsimLevelGeom& g) { return ceil_div(g.w, kSsimTileW); }
+HFC_HD int ssim_bwd_stage_rows(const SsimLevelGeom& g) { return kSsimTileH + g.wh - 1; }
+HFC_HD int ssim_bwd_stage_cols(const SsimLevelGeom& g) { return kSsimTileW + g.ww - 1; }
 
 }  // namespace hfc

@@ -10,7 +10,8 @@ smoothed (with the reference's warning), ``ms_ssim`` pools with ``avg_pool2d(ker
 tensors it returns a per-image float64 tensor computed on the device.  ``ssim`` / ``ms_ssim`` take fp32 CUDA tensors and
 return CUDA tensors without synchronising with the host.  What the kernels do not implement raises instead of falling
 back: CPU tensors ``RuntimeError``; other dtypes, 5-D inputs, windows longer than 31 taps, more than 8 levels and inputs
-that require a gradient ``NotImplementedError`` (these functions are forward-only).
+that require a gradient ``NotImplementedError`` (these functions are forward-only; ``helpers.metrics_autograd`` has the
+same API with gradients).
 """
 import warnings
 
@@ -69,7 +70,7 @@ def _require_cuda(X, Y, what):
         raise RuntimeError(f"{what}: inputs must be CUDA tensors (there is no CPU implementation)")
 
 
-def _check_supported(X, Y, win_size, what):
+def _check_supported(X, Y, win_size, what, forward_only=True):
     if X.dim() == 5:
         raise NotImplementedError(f"{what}: 5-d (conv3d) inputs are not implemented")
     _require_cuda(X, Y, what)
@@ -77,7 +78,14 @@ def _check_supported(X, Y, win_size, what):
         raise NotImplementedError(f"{what}: float32 inputs only, got {X.dtype}")
     if win_size > MAX_WIN:
         raise NotImplementedError(f"{what}: window size {win_size} > {MAX_WIN}")
-    _no_grad_check(X, Y, what)
+    if forward_only:
+        _no_grad_check(X, Y, what)
+
+
+def _no_window_grad(win, what):
+    if win is not None and torch.is_grad_enabled() and win.requires_grad:
+        raise NotImplementedError(f"{what}: no gradient with respect to the window; pass a window that does not require "
+                                  "a gradient")
 
 
 _taps_cache = {}
@@ -117,22 +125,9 @@ def _constants(K, data_range):
     return float((K1 * data_range) ** 2), float((K2 * data_range) ** 2)
 
 
-def ssim(X, Y, data_range=255, size_average=True, win_size=11, win_sigma=1.5, win=None, K=(0.01, 0.03),
-         nonnegative_ssim=False):
-    r"""SSIM of two batches of images (N, C, H, W), fp32 CUDA tensors.
-
-    Args:
-        X, Y (torch.Tensor): images
-        data_range (float or int): value range of the images (usually 1.0 or 255)
-        size_average (bool): average over the batch to a scalar; otherwise one value per image
-        win_size (int): Gaussian window length (odd)
-        win_sigma (float): Gaussian window sigma
-        win (torch.Tensor, optional): (C, 1, 1, win) window taps; overrides win_size / win_sigma
-        K (tuple): constants (K1, K2)
-        nonnegative_ssim (bool): relu the per-channel SSIM
-    Returns:
-        torch.Tensor: SSIM (0-d) or (N,)
-    """
+def _ssim_inputs(X, Y, data_range, win_size, win_sigma, win, K, forward_only):
+    """ssim(): the reference's validation in its order, then this module's limits, the warning, taps and constants.
+    Returns (X, Y, taps, c1, c2)."""
     if not X.shape == Y.shape:
         raise ValueError("Input images should have the same dimensions.")
     X, Y = _squeeze(X, Y)
@@ -144,29 +139,18 @@ def ssim(X, Y, data_range=255, size_average=True, win_size=11, win_sigma=1.5, wi
         win_size = win.shape[-1]
     if not (win_size % 2 == 1):
         raise ValueError("Window size should be odd.")
-    _check_supported(X, Y, win_size, "ssim")
+    _check_supported(X, Y, win_size, "ssim", forward_only)
+    if not forward_only:
+        _no_window_grad(win, "ssim")
     _warn_unsmoothed(X.shape, win_size)
     taps = _device_taps(win, win_size, win_sigma, X.shape[1], X.device)
     c1, c2 = _constants(K, data_range)
-    return ops.ssim_levels(X, Y, taps, c1, c2, [1.0], bool(nonnegative_ssim), size_average)
+    return X, Y, taps, c1, c2
 
 
-def ms_ssim(X, Y, data_range=255, size_average=True, win_size=11, win_sigma=1.5, win=None, weights=None,
-            K=(0.01, 0.03)):
-    r"""MS-SSIM of two batches of images (N, C, H, W), fp32 CUDA tensors.
-
-    Args:
-        X, Y (torch.Tensor): images
-        data_range (float or int): value range of the images (usually 1.0 or 255)
-        size_average (bool): average over the batch to a scalar; otherwise one value per image
-        win_size (int): Gaussian window length (odd)
-        win_sigma (float): Gaussian window sigma
-        win (torch.Tensor, optional): (C, 1, 1, win) window taps; overrides win_size / win_sigma
-        weights (list, optional): per-level weights; their number is the number of levels
-        K (tuple): constants (K1, K2)
-    Returns:
-        torch.Tensor: MS-SSIM (0-d) or (N,)
-    """
+def _ms_ssim_inputs(X, Y, data_range, win_size, win_sigma, win, weights, K, forward_only):
+    """ms_ssim(): the reference's validation in its order (dtype before dimensions, the size assert), then this module's
+    limits, the per-level warnings, taps and constants.  Returns (X, Y, taps, c1, c2, weights)."""
     if not X.shape == Y.shape:
         raise ValueError("Input images should have the same dimensions.")
     X, Y = _squeeze(X, Y)
@@ -186,13 +170,56 @@ def ms_ssim(X, Y, data_range=255, size_average=True, win_size=11, win_sigma=1.5,
     weights = [float(w) for w in torch.tensor(weights, dtype=torch.float32).reshape(-1).tolist()]
     if len(weights) > MAX_LEVELS:
         raise NotImplementedError(f"ms_ssim: at most {MAX_LEVELS} levels, got {len(weights)}")
-    _check_supported(X, Y, win_size, "ms_ssim")
+    _check_supported(X, Y, win_size, "ms_ssim", forward_only)
+    if not forward_only:
+        _no_window_grad(win, "ms_ssim")
     shape = X.shape
     for level in range(len(weights)):
         _warn_unsmoothed(shape, win_size)
         shape = torch.Size((shape[0], shape[1], (shape[2] + 1) // 2, (shape[3] + 1) // 2))
     taps = _device_taps(win, win_size, win_sigma, X.shape[1], X.device)
     c1, c2 = _constants(K, data_range)
+    return X, Y, taps, c1, c2, weights
+
+
+def ssim(X, Y, data_range=255, size_average=True, win_size=11, win_sigma=1.5, win=None, K=(0.01, 0.03),
+         nonnegative_ssim=False):
+    r"""SSIM of two batches of images (N, C, H, W), fp32 CUDA tensors.
+
+    Args:
+        X, Y (torch.Tensor): images
+        data_range (float or int): value range of the images (usually 1.0 or 255)
+        size_average (bool): average over the batch to a scalar; otherwise one value per image
+        win_size (int): Gaussian window length (odd)
+        win_sigma (float): Gaussian window sigma
+        win (torch.Tensor, optional): (C, 1, 1, win) window taps; overrides win_size / win_sigma
+        K (tuple): constants (K1, K2)
+        nonnegative_ssim (bool): relu the per-channel SSIM
+    Returns:
+        torch.Tensor: SSIM (0-d) or (N,)
+    """
+    X, Y, taps, c1, c2 = _ssim_inputs(X, Y, data_range, win_size, win_sigma, win, K, forward_only=True)
+    return ops.ssim_levels(X, Y, taps, c1, c2, [1.0], bool(nonnegative_ssim), size_average)
+
+
+def ms_ssim(X, Y, data_range=255, size_average=True, win_size=11, win_sigma=1.5, win=None, weights=None,
+            K=(0.01, 0.03)):
+    r"""MS-SSIM of two batches of images (N, C, H, W), fp32 CUDA tensors.
+
+    Args:
+        X, Y (torch.Tensor): images
+        data_range (float or int): value range of the images (usually 1.0 or 255)
+        size_average (bool): average over the batch to a scalar; otherwise one value per image
+        win_size (int): Gaussian window length (odd)
+        win_sigma (float): Gaussian window sigma
+        win (torch.Tensor, optional): (C, 1, 1, win) window taps; overrides win_size / win_sigma
+        weights (list, optional): per-level weights; their number is the number of levels
+        K (tuple): constants (K1, K2)
+    Returns:
+        torch.Tensor: MS-SSIM (0-d) or (N,)
+    """
+    X, Y, taps, c1, c2, weights = _ms_ssim_inputs(X, Y, data_range, win_size, win_sigma, win, weights, K,
+                                                  forward_only=True)
     return ops.ssim_levels(X, Y, taps, c1, c2, weights, True, size_average)
 
 

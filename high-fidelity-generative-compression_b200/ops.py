@@ -6,6 +6,7 @@ import ctypes
 from dataclasses import dataclass, replace
 
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 from ._lib import (ACT_LEAKY02, ACT_NONE, ACT_RELU, OUT_NCHW_F32, OUT_NHWC_F16, OUT_NHWC_F32,
@@ -682,18 +683,15 @@ def _metrics_ws(key, need, device):
     return buf, buf.numel() * 8
 
 
-def ssim_levels(x, y, taps, c1, c2, weights, relu_last, size_average):
-    """x, y (N, C, H, W) fp32 CUDA; taps (C, win) fp32 on x's device.  len(weights) SSIM levels (2x2 average pool in
-    between) -> prod_l value_l ** weights[l] per plane, averaged over (N, C) (0-d tensor) or over C per image ((N,)).
-    len(weights) + 1 launches, no synchronisation."""
-    assert x.is_cuda and x.dtype == torch.float32 and x.dim() == 4 and y.shape == x.shape and y.dtype == x.dtype
-    x, y = x.contiguous(), y.contiguous()
+def _ssim_forward_launches(x, y, taps, c1, c2, weights, relu_last, size_average, ws, ws_bytes):
+    """The level and finalize launches of ssim_levels on workspace `ws`.  Returns (out, pyramid): pyramid[l] is level l's
+    input pair (x, y at level 0, then the pooled planes the level kernels wrote)."""
     n, c, h, w = x.shape
     win = taps.shape[-1]
-    assert taps.is_cuda and taps.dtype == torch.float32 and taps.is_contiguous() and tuple(taps.shape) == (c, win)
     levels = len(weights)
-    ws, ws_bytes = _metrics_ws("ssim", int(lib.hfc_ssim_ws_bytes(n, c, h, w, win, levels)), x.device)
+    pyramid = []
     for level in range(levels):
+        pyramid.append((x, y))
         if level < levels - 1:
             hp, wp = (x.shape[2] + 1) // 2, (x.shape[3] + 1) // 2
             px = torch.empty((n, c, hp, wp), dtype=torch.float32, device=x.device)
@@ -707,7 +705,99 @@ def ssim_levels(x, y, taps, c1, c2, weights, relu_last, size_average):
     wts = (ctypes.c_float * levels)(*weights)
     check(lib.hfc_ssim_finalize(n, c, h, w, win, levels, wts, int(bool(relu_last)), int(bool(size_average)), _ptr(ws),
                                 ws_bytes, _ptr(out), _stream()), "ssim_finalize")
-    return out.reshape(()) if size_average else out
+    return (out.reshape(()) if size_average else out), pyramid
+
+
+def _ssim_backward_launches(pyramid, taps, c1, c2, weights, relu_last, size_average, ws, ws_bytes, grad_out, need_x,
+                            need_y):
+    """Gradients of ssim_levels' output w.r.t. pyramid[0] from the forward's workspace (its per-plane level sums) and
+    the kept pyramid: one coefficient launch, then per level (coarsest first) a gradient-map and a level-backward launch.
+    Returns (dx, dy), None where not needed."""
+    x, y = pyramid[0]
+    n, c, h, w = x.shape
+    win = taps.shape[-1]
+    levels = len(weights)
+    dev = x.device
+    g = grad_out.to(dtype=torch.float32).contiguous()
+    coef = torch.empty(n * c * levels * 2, dtype=torch.float32, device=dev)
+    wts = (ctypes.c_float * levels)(*weights)
+    check(lib.hfc_ssim_grad_coeffs(n, c, h, w, win, levels, wts, int(bool(relu_last)), int(bool(size_average)), _ptr(ws),
+                                   ws_bytes, _ptr(g), _ptr(coef), _stream()), "ssim_grad_coeffs")
+    maps_bytes = int(lib.hfc_ssim_grad_maps_bytes(n, c, h, w, win, levels))
+    if maps_bytes < 0:
+        raise _lib.HfcError(f"libhfc ssim_grad_maps_bytes failed: {lib.hfc_last_error().decode('utf-8', 'replace')}")
+    maps = torch.empty(max(4, maps_bytes // 4), dtype=torch.float32, device=dev)
+    dx = dy = None
+    for level in reversed(range(levels)):
+        xl, yl = pyramid[level]
+        check(lib.hfc_ssim_grad_maps(_ptr(xl), _ptr(yl), n, c, h, w, level, levels, _ptr(taps), win, c1, c2, _ptr(coef),
+                                     _ptr(maps), maps.numel() * 4, _stream()), "ssim_grad_maps")
+        gx = torch.empty_like(xl) if need_x else None
+        gy = torch.empty_like(yl) if need_y else None
+        check(lib.hfc_ssim_level_bwd(_ptr(xl), _ptr(yl), _ptr(maps), n, c, h, w, level, _ptr(taps), win, _ptr(dx),
+                                     _ptr(dy), _ptr(gx), _ptr(gy), _stream()), "ssim_level_bwd")
+        dx, dy = gx, gy
+    return dx, dy
+
+
+def _ssim_check_args(x, y, taps):
+    assert x.is_cuda and x.dtype == torch.float32 and x.dim() == 4 and y.shape == x.shape and y.dtype == x.dtype
+    win = taps.shape[-1]
+    assert taps.is_cuda and taps.dtype == torch.float32 and taps.is_contiguous() and tuple(taps.shape) == (x.shape[1], win)
+
+
+def ssim_levels(x, y, taps, c1, c2, weights, relu_last, size_average):
+    """x, y (N, C, H, W) fp32 CUDA; taps (C, win) fp32 on x's device.  len(weights) SSIM levels (2x2 average pool in
+    between) -> prod_l value_l ** weights[l] per plane, averaged over (N, C) (0-d tensor) or over C per image ((N,)).
+    len(weights) + 1 launches, no synchronisation."""
+    _ssim_check_args(x, y, taps)
+    x, y = x.contiguous(), y.contiguous()
+    n, c, h, w = x.shape
+    ws, ws_bytes = _metrics_ws("ssim", int(lib.hfc_ssim_ws_bytes(n, c, h, w, taps.shape[-1], len(weights))), x.device)
+    return _ssim_forward_launches(x, y, taps, c1, c2, weights, relu_last, size_average, ws, ws_bytes)[0]
+
+
+class SsimLevelsFn(torch.autograd.Function):
+    """ssim_levels with a gradient w.r.t. x and y.  The forward runs ssim_levels' launches (bit-identical values) on a
+    workspace of its own, so that a second forward before this one's backward cannot overwrite the per-plane level sums
+    the backward reads; it keeps the pooled pyramid.  taps, c1, c2, weights and the flags are constants."""
+
+    @staticmethod
+    def forward(ctx, x, y, taps, c1, c2, weights, relu_last, size_average):
+        _ssim_check_args(x, y, taps)
+        xc, yc = x.contiguous(), y.contiguous()
+        n, c, h, w = xc.shape
+        need = int(lib.hfc_ssim_ws_bytes(n, c, h, w, taps.shape[-1], len(weights)))
+        if need < 0:
+            raise _lib.HfcError(f"libhfc ssim workspace query failed: {lib.hfc_last_error().decode('utf-8', 'replace')}")
+        ws = torch.empty(max(1, (need + 7) // 8), dtype=torch.float64, device=xc.device)
+        out, pyramid = _ssim_forward_launches(xc, yc, taps, c1, c2, weights, relu_last, size_average, ws, ws.numel() * 8)
+        ctx.save_for_backward(x, y)
+        ctx.pooled = pyramid[1:]
+        ctx.ws = ws
+        ctx.consts = (taps, c1, c2, list(weights), relu_last, size_average)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        need_x, need_y = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        if not (need_x or need_y):
+            return (None,) * 8
+        x, y = ctx.saved_tensors
+        taps, c1, c2, weights, relu_last, size_average = ctx.consts
+        pyramid = [(x.contiguous(), y.contiguous())] + ctx.pooled
+        dx, dy = _ssim_backward_launches(pyramid, taps, c1, c2, weights, relu_last, size_average, ctx.ws,
+                                         ctx.ws.numel() * 8, grad_out, need_x, need_y)
+        return dx, dy, None, None, None, None, None, None
+
+
+def ssim_levels_grad(x, y, taps, c1, c2, weights, relu_last, size_average):
+    """ssim_levels, differentiable w.r.t. x and y when grad mode is on and either requires a gradient (SsimLevelsFn);
+    otherwise ssim_levels itself.  Backward: at most 2 * len(weights) + 1 launches, no synchronisation."""
+    if torch.is_grad_enabled() and (x.requires_grad or y.requires_grad):
+        return SsimLevelsFn.apply(x, y, taps, c1, c2, list(weights), relu_last, size_average)
+    return ssim_levels(x, y, taps, c1, c2, weights, relu_last, size_average)
 
 
 def psnr(a, b, max_val=255.0):

@@ -483,6 +483,28 @@ int hfc_ssim_level(const float* x, const float* y, int32_t n, int32_t c, int32_t
                    int64_t ws_bytes, void* stream);
 int hfc_ssim_finalize(int32_t n, int32_t c, int32_t h0, int32_t w0, int32_t win, int32_t levels, const float* weights_host,
                       int32_t relu_last, int32_t size_average, void* ws, int64_t ws_bytes, float* out, void* stream);
+/* Backward of the above (metrics.py:66-103 _ssim, 150-161 ssim's reductions, 214-236 ms_ssim's relu / pow / prod /
+ * mean): 2 * levels + 1 launches, coarsest level first, no float atomics (bit-reproducible, independent of the batch).
+ * hfc_ssim_grad_coeffs: reads the per-plane level sums that hfc_ssim_finalize left in ws (the same ws, untouched since)
+ * and the upstream gradient grad_out on the device (out's shape: [1] with size_average, else [n]); writes coeffs
+ * [n * c][levels][2] fp32 (the weight of each valid output's ssim and cs at that level).  A level clamped by its relu gets
+ * exactly 0, and so does every level of a plane where one level is clamped.
+ * hfc_ssim_grad_maps: per level, on that level's inputs x, y (the forward's pooled planes): the four gradient maps
+ * (d mu1, d mu2, d sigma^2 terms, d E[xy]) per valid output, fp32x4, into maps (16-byte aligned, at least
+ * hfc_ssim_grad_maps_bytes(n, c, h0, w0, win, levels) bytes, which covers every level; one buffer serves all levels).
+ * hfc_ssim_level_bwd: the level's input gradients from its maps, plus 0.25 x the next level's input gradient
+ * (dx_coarse / dy_coarse, (n, c, h_{l+1}, w_{l+1}); NULL at the last level) at the pooled pixel each input pixel fed.
+ * dx or dy may be NULL when not needed; level 0 writes the gradients of the caller's x and y. */
+int64_t hfc_ssim_grad_maps_bytes(int32_t n, int32_t c, int32_t h0, int32_t w0, int32_t win, int32_t levels);
+int hfc_ssim_grad_coeffs(int32_t n, int32_t c, int32_t h0, int32_t w0, int32_t win, int32_t levels,
+                         const float* weights_host, int32_t relu_last, int32_t size_average, const void* ws,
+                         int64_t ws_bytes, const float* grad_out, float* coeffs, void* stream);
+int hfc_ssim_grad_maps(const float* x, const float* y, int32_t n, int32_t c, int32_t h0, int32_t w0, int32_t level,
+                       int32_t levels, const float* taps, int32_t win, float c1, float c2, const float* coeffs,
+                       float* maps, int64_t maps_bytes, void* stream);
+int hfc_ssim_level_bwd(const float* x, const float* y, const float* maps, int32_t n, int32_t c, int32_t h0, int32_t w0,
+                       int32_t level, const float* taps, int32_t win, const float* dx_coarse, const float* dy_coarse,
+                       float* dx, float* dy, void* stream);
 /* PSNR (metrics.py:7-18): out[i] = 20 log10(max_val) - 10 log10(mean over image i of (a - b)^2), fp64 throughout;
  * per_image = c * h * w.  ws: device scratch of at least hfc_psnr_ws_bytes(n, per_image) bytes.  Two launches. */
 int64_t hfc_psnr_ws_bytes(int32_t n, int64_t per_image);
